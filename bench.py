@@ -141,7 +141,12 @@ class SumcheckWorkload:
         dp.lib().dp_synchronize()
 
     def step_resident(self, i):
-        return self.dp.sumcheck_prove_parallel(self.dev_sets[i % self.NSETS], self.products, self.NV)
+        self.last = self.dp.sumcheck_prove_parallel(self.dev_sets[i % self.NSETS], self.products, self.NV)
+        return self.last
+
+    def outputs(self):
+        point, msgs, fin = self.last
+        return {"point": point, "msgs": msgs, "final_evals": fin}
 
     def step_e2e(self, i):
         ms = [self.dp.Mle.upload(a, False) for a in self.host_sets[i % self.NSETS]]
@@ -195,7 +200,11 @@ class BasefoldWorkload:
         self.d2h = int(flat.size * 8)
 
     def step_resident(self, i):
-        self.dp.pcs_open(self.mle, self.NV, self.point, cap=1 << 23)
+        self.last = self.dp.pcs_open(self.mle, self.NV, self.point, cap=1 << 23)
+
+    def outputs(self):
+        root, flat = self.last
+        return {"root": root, "proof": flat}
 
     def step_e2e(self, i):
         m = self.dp.Mle.upload(self.evals, False)
@@ -281,6 +290,9 @@ class DenseWorkload:
     def run_e2e(self, k, device):
         self.ctx.prove_concurrent(host_workers(self.STREAMS), k * self.units_per_step, device=device, e2e=True)
 
+    def outputs(self):
+        return {"proof": self.ctx.last_concurrent_proof()}
+
     def cpu_step(self, O, i):
         _, ms = O.zkml_prove(self.NL, self.W, self.SEED_MODEL, self.SEED_INPUT, want_proof=False)
         return ms[1] * 1e-3     # Prover::prove only; Context::generate (ms[0]) is setup
@@ -340,6 +352,9 @@ class CnnWorkload:
 
     def run_e2e(self, k, device):
         self.ctx.prove_concurrent(host_workers(self.STREAMS), k * self.units_per_step, device=device, e2e=True)
+
+    def outputs(self):
+        return {"proof": self.ctx.last_concurrent_proof()}
 
     def cpu_step(self, O, i):
         _, ms = O.model_prove(self.desc, self.data, self.x, want_proof=False)
@@ -430,6 +445,25 @@ def max_over_ranks(ms, dist, device="cuda"):
 def whole_job_value(units_per_rank, world, ms):
     """replicas: every rank processes `units_per_rank` independent units; value = all units / slowest rank's time"""
     return units_per_rank * world / (ms * 1e-3)
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(outdir, outputs):
+    """outputs: {workload: {name: uint64 array}} -> outdir/<workload>_<name>.npy.  Every 64-bit field word is stored exactly as
+    two float64 values, its low and high 32 bits, along a new last axis of size 2."""
+    arrays = {}
+    for wk, outs in outputs.items():
+        for name, a in outs.items():
+            a = np.asarray(a, dtype=np.uint64)
+            arrays["%s_%s" % (wk, name)] = np.stack([a & np.uint64(0xFFFFFFFF), a >> np.uint64(32)], axis=-1).astype(np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit("bench.py: outputs take %d bytes, more than the %d-byte limit of --dump-outputs" % (total, DUMP_LIMIT))
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(outdir, name + ".npy"), a)
 
 
 # ---- CPU arm -----------------------------------------------------------------------------------------
@@ -613,6 +647,7 @@ def run_gpu_workload(env, wl, K, W, full):
         dp.set_wait_mode(1)      # many proofs in flight: proving threads sleep on the library's poller instead of spinning (DESIGN.md section 5)
         with clk:
             ms, launches = timed_many(wl.run_resident, K, W)
+        outputs = wl.outputs()   # the last timed step's result, before the legs below overwrite it
         ms_e2e, _ = timed_many(wl.run_e2e, K, 1)
         if full:
             dp.set_wait_mode(0)  # one proof at a time: the single proving thread spins (lowest latency)
@@ -622,6 +657,7 @@ def run_gpu_workload(env, wl, K, W, full):
     else:
         with clk:
             ms, launches = timed(wl.step_resident, K, W)
+        outputs = wl.outputs()
         ms_e2e, _ = timed(wl.step_e2e, K, 2)
     clocks = clk.summary()
 
@@ -658,7 +694,8 @@ def run_gpu_workload(env, wl, K, W, full):
     res = {"metric": wl.metric, "value": v, "unit": wl.unit, "steps": K, "warmup": W, "ms_per_step": ms / K,
            "e2e": {"value": whole_job_value(K * ups, world, ms_e2e), "unit": wl.unit, "h2d_bytes_per_step": wl.h2d * ups, "d2h_bytes_per_step": wl.d2h * ups},
            "gpu_launches": int(launches), "units_per_step": ups, "single_stream_latency_ms": latency_ms,
-           "alg_GBps_whole_step": wl.alg_bytes * v / world / 1e9, "workload": wl.name, "l2": wl.l2_note, "clocks": clocks}
+           "alg_GBps_whole_step": wl.alg_bytes * v / world / 1e9, "workload": wl.name, "l2": wl.l2_note, "clocks": clocks,
+           "outputs": outputs}
     if hasattr(wl, "field_ops"):
         res["field_ops_per_s"] = wl.field_ops * v / world
         res["hbm_frac_whole_proof"] = wl.alg_bytes * v / world / 1e9 / peaks["hbm_gbs"]
@@ -799,7 +836,10 @@ def main():
     ap.add_argument("--workload", default="dense4m", choices=list(WORKLOADS))
     ap.add_argument("--only", action="store_true", help="measure only --workload (skip the other BASELINE workloads)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of each measured workload computed to DIR/<workload>_<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -849,6 +889,7 @@ def main():
     wl = WORKLOADS[args.workload]()
     K = args.steps if args.steps is not None else {"dense4m": 6, "cnn264k": 6, "sumcheck20": 20, "basefold24": 5}[args.workload]
     head = run_gpu_workload(env, wl, K, max(W, 3), True)
+    outputs = {args.workload: head.pop("outputs")}
     extra = {}
     for k in others:
         if world > 1 and k in ("sumcheck20", "basefold24"):
@@ -856,6 +897,7 @@ def main():
         w2 = WORKLOADS[k]()
         k2 = min(K, {"dense4m": 6, "cnn264k": 6, "sumcheck20": 20, "basefold24": 5}[k])
         r2 = run_gpu_workload(env, w2, k2, 3, False)
+        outputs[k] = r2.pop("outputs")
         r2.pop("clocks", None)
         if r2.get("roofline"):
             r2["roofline"].pop("kernels", None)     # the per-kernel tables are printed for the headline workload only
@@ -896,6 +938,8 @@ def main():
         for k in ("field_ops_per_s", "hbm_frac_whole_proof", "poseidon2_perm_per_s", "pipe_frac_whole_step", "parity_error"):
             if k in head:
                 out[k] = head[k]
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(out))
     if dist is not None:
         dist.destroy_process_group()

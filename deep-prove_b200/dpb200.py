@@ -516,6 +516,14 @@ class ZkmlContext:
         hcheck(H.dph_zkml_prove_concurrent(self.h, int(device), int(n_workers), int(n_proofs), int(bool(e2e)), label, C.byref(sec)))
         return sec.value
 
+    def last_concurrent_proof(self):
+        """flat proof (as prove() returns it) of the job claimed last in the most recent prove_concurrent call"""
+        H = host()
+        H.dph_zkml_last_concurrent_proof.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
+        n = C.c_uint64()
+        hcheck(H.dph_zkml_last_concurrent_proof(self.h, _ptr(self._out), self._out.size, C.byref(n)))
+        return self._out[: n.value].copy()
+
     def free(self):
         if self.h:
             host().dph_zkml_context_free(self.h)

@@ -213,11 +213,14 @@ struct ZkPool {
     // proofs this pool has already run -- the first call of a pool is not staggered): latency-bound and GPU-bound phases of
     // different proofs then overlap.  The ramp-up and ramp-down this costs are inside the caller's timed region.
     uint32_t active = 0; uint64_t call_gen = 0; double stagger_s = 0.0, avg_proof_s = 0.0; uint64_t n_timed = 0;
+    // the proof of the job claimed last in the most recent call; every other proof of a call is dropped
+    dp::zkml::Proof last; bool has_last = false;
+    void keep_last(dp::zkml::Proof &p) { std::lock_guard<std::mutex> lk(mu); last = std::move(p); has_last = true; }
     void worker(uint32_t idx) {
         bool inited = false; uint64_t seen_gen = 0;
         for (;;) {
-            uint64_t gen; double delay = 0.0;
-            { std::unique_lock<std::mutex> lk(mu); cv.wait(lk, [&] { return stop || (pending > 0 && idx < active); }); if (stop) break; pending--; inflight++; gen = call_gen; if (gen != seen_gen) { seen_gen = gen; delay = stagger_s * idx; } }
+            uint64_t gen; double delay = 0.0; bool last_job;
+            { std::unique_lock<std::mutex> lk(mu); cv.wait(lk, [&] { return stop || (pending > 0 && idx < active); }); if (stop) break; pending--; inflight++; last_job = pending == 0; gen = call_gen; if (gen != seen_gen) { seen_gen = gen; delay = stagger_s * idx; } }
             try {
                 const bool first_ever = !inited;     // grows this thread's device arena: not a representative duration
                 if (!inited) { dp::check(dp_init(device)); inited = true; }
@@ -230,7 +233,8 @@ struct ZkPool {
                     dp::zkml::Proof p = prover.prove(h->trace_input);
                     std::vector<uint64_t> bytes = p.flatten(h->model.nodes.size());
                     if (bytes.empty()) throw dp::Error(DP_ERR_STATE, "empty proof");
-                } else { dp::zkml::Proof p = prover.prove(h->trace); (void)p; }
+                    if (last_job) keep_last(p);
+                } else { dp::zkml::Proof p = prover.prove(h->trace); if (last_job) keep_last(p); }
                 const double sec = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
                 if (getenv("DP_HOST_PROF") && idx == 0) { struct timespec cts1; clock_gettime(CLOCK_THREAD_CPUTIME_ID, &cts1);
                     fprintf(stderr, "[worker0] proof wall %.2f ms, thread CPU %.2f ms, transcript permutations %llu\n", sec * 1e3, (cts1.tv_sec - cts0.tv_sec) * 1e3 + (cts1.tv_nsec - cts0.tv_nsec) * 1e-6, (unsigned long long)t.permutations()); }
@@ -257,7 +261,7 @@ extern "C" int dph_zkml_prove_concurrent(void *handle, int device, uint32_t n_wo
     auto t0 = std::chrono::steady_clock::now();
     {
         std::lock_guard<std::mutex> lk(pool->mu);
-        pool->label = label; pool->failed = false; pool->e2e = e2e != 0; pool->pending = n_proofs; pool->active = n_workers; pool->call_gen++;
+        pool->label = label; pool->failed = false; pool->has_last = false; pool->e2e = e2e != 0; pool->pending = n_proofs; pool->active = n_workers; pool->call_gen++;
         // stagger only when every worker gets several proofs (otherwise the ramps cost more than the overlap gains)
         pool->stagger_s = (!no_stagger && n_workers > 1 && n_proofs >= 3 * n_workers && pool->n_timed > 0) ? pool->avg_proof_s / n_workers : 0.0;
     }
@@ -266,6 +270,26 @@ extern "C" int dph_zkml_prove_concurrent(void *handle, int device, uint32_t n_wo
     { std::unique_lock<std::mutex> lk(pool->mu); pool->done_cv.wait(lk, [&] { return pool->pending == 0 && pool->inflight == 0; }); }
     if (out_seconds) *out_seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
     if (pool->failed) { g_herr = pool->err; return 1; }
+    return 0;
+    DPH_CATCH
+}
+// flat proof (the dph_zkml_prove image) of the job claimed last in the most recent dph_zkml_prove_concurrent call on `handle`
+extern "C" int dph_zkml_last_concurrent_proof(void *handle, uint64_t *out, uint64_t cap, uint64_t *out_len) {
+    DPH_TRY
+    ZkHandle *h = (ZkHandle *)handle;
+    ZkPool *pool = nullptr;
+    { std::lock_guard<std::mutex> lk(g_pools_mu); auto it = g_pools.find(handle); if (it != g_pools.end()) pool = it->second.get(); }
+    const char *none = "dph_zkml_last_concurrent_proof: no completed dph_zkml_prove_concurrent call";
+    if (!pool) throw dp::Error(DP_ERR_STATE, none);
+    std::vector<uint64_t> f;
+    {
+        std::lock_guard<std::mutex> lk(pool->mu);
+        if (!pool->has_last) throw dp::Error(DP_ERR_STATE, none);
+        f = pool->last.flatten(h->model.nodes.size());
+    }
+    *out_len = f.size();
+    if (f.size() > cap) { g_herr = "dph_zkml_last_concurrent_proof: output buffer too small"; return 2; }
+    memcpy(out, f.data(), 8 * f.size());
     return 0;
     DPH_CATCH
 }

@@ -43,3 +43,7 @@ def test_proof_parity(gpu, nl, width):
     ctx.run_inference(x)
     again = ctx.prove_trace(want_proof=True)
     assert (again == exp).all()
+    # the concurrent path (bench.py's timed path) keeps the proof of its last job, from the stored trace and end to end
+    for e2e in (False, True):
+        ctx.prove_concurrent(3, 5, e2e=e2e)
+        assert (ctx.last_concurrent_proof() == exp).all()

@@ -26,14 +26,15 @@ def test_upload_canonicalises(gpu):
     assert (got == np.array([0, 1, (2**64 - 1) % P, 0, 5, P - 1, 7, 8], dtype=np.uint64)).all()
 
 
-@pytest.mark.parametrize("nv", [0, 1, 2, 5, 10, 11, 12, 13, 17])
+@pytest.mark.parametrize("nv", [0, 1, 2, 5, 10, 11, 12, 13, 17, 25])
 def test_eq_build(gpu, nv):
     r = O.splitmix_e(50 + nv, nv) if nv else np.zeros((0, 2), dtype=np.uint64)
     assert (gpu.Mle.eq(r).download() == O.build_eq(r)).all()
 
 
 @pytest.mark.parametrize("nv,k,ext", [(3, 1, False), (6, 6, True), (10, 4, False), (12, 12, False), (14, 5, True),
-                                      (16, 10, False), (16, 16, True), (20, 10, False), (20, 10, True)])
+                                      (16, 10, False), (16, 16, True), (20, 10, False), (20, 10, True),
+                                      (9, 5, False), (10, 5, True), (19, 1, False), (20, 2, True)])
 def test_fix_high(gpu, nv, k, ext):
     f = O.splitmix_e(nv * 31 + k, 1 << nv) if ext else O.splitmix_f(nv * 31 + k, 1 << nv)
     pt = O.splitmix_e(77 + k, k)
